@@ -10,6 +10,7 @@ replica and its own batch; the only collective is the final gather of the top-k 
 
   python bench.py [--gpus N --steps K --warmup W]          our CUDA path (one JSON line)
   python bench.py --impl reference ...                     the CPU path (oracle port) on host cores
+  python bench.py ... --dump-outputs DIR                    also the last timed step's outputs, DIR/<name>.npy
 
 `value`  : whole-job queries/s with the query batch already in HBM (device-timed, max over ranks)
 `e2e`    : the same metric through the host-buffer C-ABI call (dann_search_batch): pinned host
@@ -30,6 +31,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the tree as it found it (it may be read-only)
 
 import numpy as np  # noqa: E402
 
@@ -56,7 +58,13 @@ def parse_args():
     ap.add_argument("--no-secondary", action="store_true", help="skip the attached configs[1] (1M x 768, batch 1024) run")
     ap.add_argument("--mode", default="batch", choices=["batch", "scan"],
                     help="scan: per-row latency of the operator surface (rescan + gettuple x k) instead of batch QPS")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path returned in its last step as DIR/<name>.npy (float32/float64)")
     a = ap.parse_args()
+    if a.dump_outputs and a.mode == "scan":
+        ap.error("--dump-outputs covers the batch path (--mode batch) and --impl reference")
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     if not a.batch:
         a.batch = 4096 if a.n >= 10_000_000 else 1024
     return a
@@ -74,6 +82,28 @@ os.dup2(2, 1)
 
 def emit(line: dict):
     os.write(_REAL_STDOUT, (json.dumps(line) + "\n").encode())
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, arrays: dict):
+    """--dump-outputs: each array as out_dir/<name>.npy, integers as float64 (exact below 2**53; an empty tid slot,
+    ~0 as int64, reads -1).  All arrays share their leading (query) axis; when they would exceed DUMP_LIMIT bytes in
+    all, the same fixed, seeded sample of queries is kept in each and its indices are written as rows.npy."""
+    arrays = {k: np.asarray(v).astype(np.float32 if np.asarray(v).dtype == np.float32 else np.float64)
+              for k, v in arrays.items()}
+    nq = next(iter(arrays.values())).shape[0]
+    room = DUMP_LIMIT - 4096 * (len(arrays) + 1)                  # .npy headers
+    if sum(a.nbytes for a in arrays.values()) > room:
+        per_query = sum(a.nbytes for a in arrays.values()) // nq + 8
+        rows = np.sort(np.random.default_rng(0).choice(nq, room // per_query, replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+    log(f"[bench] outputs of the last timed step -> {out_dir}: " + ", ".join(f"{k}{list(a.shape)}" for k, a in arrays.items()))
 
 
 # (search_list_size, rescore) in increasing cost (visits ~ L + rescore); recall is driven mostly by rescore
@@ -320,8 +350,12 @@ def run_reference(args):
         oracle.scan_batch(snap, qs[w * sample:(w + 1) * sample], None, None, L, rescore, k, threads=threads)
     t0 = time.perf_counter()
     for s in range(args.warmup, nb):
-        oracle.scan_batch(snap, qs[s * sample:(s + 1) * sample], None, None, L, rescore, k, threads=threads)
+        res = oracle.scan_batch(snap, qs[s * sample:(s + 1) * sample], None, None, L, rescore, k, threads=threads)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        tid, dist_, count, stats = res
+        dump_outputs(args.dump_outputs, {"tid": tid.view(np.int64), "dist": dist_, "count": count,
+                                         "stats": np.stack([stats[f] for f in stats.dtype.names], 1)})
     qps = args.steps * sample / dt
     lat = cpu_latency(oracle, snap, qs[:16], L, rescore, k)
     native = native_arm(oracle, snap, qs[:sample], L, rescore, k, threads, 3.0)
@@ -345,8 +379,9 @@ def run_reference(args):
     emit(line)
 
 
-def run_ours(args, n, B, steps, warmup, device, rank, world, full=True):
-    """One measurement of our CUDA path on an n x dim index with B queries per GPU per step -> result dict (rank 0)."""
+def run_ours(args, n, B, steps, warmup, device, rank, world, full=True, dump=None):
+    """One measurement of our CUDA path on an n x dim index with B queries per GPU per step -> result dict (rank 0).
+    dump: directory for the outputs of the last timed step (dump_outputs)."""
     import torch
     import torch.distributed as dist
     from pgvectorscale_b200 import diskann
@@ -502,6 +537,12 @@ def run_ours(args, n, B, steps, warmup, device, rank, world, full=True):
                 shard.gather_packed(h_tid.to(device, non_blocking=True), h_dist.to(device, non_blocking=True), B)
         barrier()
         e2e_s = time.perf_counter() - t0
+    if dump and rank == 0:
+        gt, gd = gathered
+        out = {"tid": gt.cpu().numpy(), "dist": gd.cpu().numpy()}
+        if world == 1:      # the per-query counters, and the host-buffer call's rows for the same last-step queries
+            out.update(count=d_cnt.cpu().numpy(), stats=d_stats.cpu().numpy(), e2e_tid=h_tid.numpy(), e2e_dist=h_dist.numpy())
+        dump_outputs(dump, out)
 
     # ---- max over ranks ---------------------------------------------------------------------
     tm = torch.tensor([dev_ms, e2e_s * 1e3, search_ms, rerank_ms], dtype=torch.float64, device=device)
@@ -692,7 +733,7 @@ def main():
             raise
         except Exception as e:
             secondary = {"error": repr(e)}
-    line = run_ours(args, args.n, args.batch, args.steps, args.warmup, device, rank, world)
+    line = run_ours(args, args.n, args.batch, args.steps, args.warmup, device, rank, world, dump=args.dump_outputs)
     if rank == 0:
         if secondary is not None:
             line["secondary"] = secondary

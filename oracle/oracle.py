@@ -255,15 +255,15 @@ def native_lib():
     "not the reference's build flags").  Only scan_batch(native=True) uses it; parity always runs on the reference-flag build."""
     global _NATIVE
     if _NATIVE is None:
-        # -march=native code must never run on another machine: the file name carries this CPU's model and flags
-        import hashlib
-        ident = "".join(l for l in open("/proc/cpuinfo") if l.startswith(("model name", "flags")))[:20000]
-        tag = hashlib.sha1(ident.encode()).hexdigest()[:10]
-        so = os.path.join(_HERE, f"liboracle_native_{tag}.so")
-        src = [os.path.join(_HERE, f) for f in ("oracle.cpp", "oracle.h", "Makefile")]
-        if not os.path.exists(so) or any(os.path.getmtime(x) > os.path.getmtime(so) for x in src):
-            subprocess.run(["make", "-C", _HERE, "-s", "native", f"NATIVE_SO={os.path.basename(so)}"], check=True,
-                           stdout=subprocess.DEVNULL)
+        # -march=native code must never run on another machine, and the tree may be read-only: built per process in a
+        # temporary directory, removed at exit
+        import atexit
+        import shutil
+        import tempfile
+        tmp = tempfile.mkdtemp(prefix="dann_oracle_native_")
+        atexit.register(shutil.rmtree, tmp, True)
+        so = os.path.join(tmp, "liboracle_native.so")
+        subprocess.run(["make", "-C", _HERE, "-s", "native", f"NATIVE_SO={so}"], check=True, stdout=subprocess.DEVNULL)
         _NATIVE = C.CDLL(so)
     return _NATIVE
 

@@ -20,6 +20,18 @@ def lib(lib_built):
     return diskann
 
 
+@pytest.fixture
+def sock_dir():
+    """A short directory for the sidecar's Unix-domain socket: a socket path holds at most 107 bytes, which a deep
+    tmp_path (a long TMPDIR, xdist's per-worker directories) can exceed."""
+    import os
+    import shutil
+    import tempfile
+    d = tempfile.mkdtemp(prefix="dann", dir="/tmp" if os.path.isdir("/tmp") else None)
+    yield d
+    shutil.rmtree(d, ignore_errors=True)
+
+
 def test_coalescer_concurrent_single_query_callers_get_private_scan_results(lib):
     """SURVEY §8f row 4: many blocking single-query callers (backends) -> few batch calls; every caller gets exactly
     what the oracle's private scan of its query returns, whatever it was batched with."""
@@ -98,7 +110,7 @@ def test_c_load_generator_through_the_coalescer(lib, lib_built, tmp_path):
     assert chk == d["tid_checksum"]
 
 
-def test_sidecar_process_serves_concurrent_backends(lib, lib_built, tmp_path):
+def test_sidecar_process_serves_concurrent_backends(lib, lib_built, tmp_path, sock_dir):
     """sidecar/dann_sidecar.c: one process owns the index, every connection is a backend; concurrent clients get
     exactly the oracle's private scans (rows, distance bits, counters), keyed and unkeyed."""
     import os
@@ -120,7 +132,7 @@ def test_sidecar_process_serves_concurrent_backends(lib, lib_built, tmp_path):
                     "-Wl,-rpath," + libdir, "-lpthread", "-o", exe], check=True)
     s = build_case(1200, 48, COSINE, seed=12, kind="normal", R=24, L_build=48, labels=True, deleted_every=10)
     s.save_raw(str(tmp_path / "snap.raw"))
-    sock = str(tmp_path / "dann.sock")
+    sock = os.path.join(sock_dir, "dann.sock")
     proc = subprocess.Popen([exe, str(tmp_path / "snap.raw"), sock, "32", "20000"], stderr=subprocess.PIPE, text=True)
     try:
         for _ in range(600):
@@ -184,7 +196,7 @@ def test_sidecar_process_serves_concurrent_backends(lib, lib_built, tmp_path):
     assert "queries in" in proc.stderr.read()
 
 
-def test_sidecar_cold_start_from_relation_files_and_staleness_signal(lib, lib_built, tmp_path):
+def test_sidecar_cold_start_from_relation_files_and_staleness_signal(lib, lib_built, tmp_path, sock_dir):
     """dann_sidecar --relation: index pages (dann_pg_extract_sbq) + the table's vector column from its heap and TOAST
     files (dann_pg_heap_fetch_vectors) -> the served index; scans equal the oracle's on the snapshot the files were
     written from.  SIGHUP re-reads the page headers: unchanged -> keeps serving; a page LSN moved -> exits with status 5."""
@@ -213,7 +225,7 @@ def test_sidecar_cold_start_from_relation_files_and_staleness_signal(lib, lib_bu
     dead = (s.heap_tid & np.uint64(0xFFFF)) == 0               # vacuumed nodes keep their invalid heap pointer
     s.heap_tid = np.where(dead, htids & np.uint64(0xFFFFFFFFFFFF0000), htids)
     meta, _, _ = pgpages.write_index(s, ipath)
-    sock = str(tmp_path / "pg.sock")
+    sock = os.path.join(sock_dir, "pg.sock")
     args = [exe, "--relation", ipath, hpath, tpath, sock, "dim=768", f"R={s.R}", "bits=%d" % s.bits, "distance=0",
             "start=%d:%d" % meta["start"], "means=%d:%d" % meta["means"], "atts=8d", "max_batch=16", "max_wait_us=2000"]
     proc = subprocess.Popen(args, stderr=subprocess.PIPE, text=True)

@@ -84,16 +84,16 @@ def run(args, device, log):
     X = torch.empty((n, dim), dtype=torch.float32, device=device)
     fx.fill_rows(X, n, dim, args.data, device)
     idx.set_vectors_device(X.data_ptr())
-    nq = 200
+    nq = args.warmup + args.steps          # one step = one scan
     q = fx.gen_queries(nq, 1, dim, args.data, device).cpu().numpy()
     rows = fx.SparseRows(n, dim)
     snap.vectors = rows.arr
     rows.fill_from_device(fx.oracle_rerank_rows(oracle, snap, q, L, rescore, k, fx.host_cores()["effective"]), X)
-    m = measure(idx, snap, oracle, q, L, rescore, k)
+    m = measure(idx, snap, oracle, q, L, rescore, k, warm=args.warmup)
     line = {"metric": f"index-scan operator latency (amrescan + {k} x amgettuple), {n}x{dim}-d SBQ diskann index",
-            "mode": "scan", "unit": "ms", "higher_is_better": False, "n_gpus": 1,
+            "mode": "scan", "unit": "ms", "higher_is_better": False, "n_gpus": 1, "steps": args.steps, "warmup": args.warmup,
             "value": m["gettuple"]["scan_of_k_rows_ms"]["p50"],
-            "config": {"workload": f"{n}x{dim}-d, one scan at a time, search_list_size={L}, rescore={rescore}, k={k}, {nq - 20} timed scans"}}
+            "config": {"workload": f"{n}x{dim}-d, one scan at a time, search_list_size={L}, rescore={rescore}, k={k}, {args.steps} timed scans"}}
     line.update({kk: v for kk, v in m.items() if kk not in ("scans", "search_list_size", "rescore", "k")})
     idx.close()
     return line
