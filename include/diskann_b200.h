@@ -151,8 +151,9 @@ void dann_scan_end(dann_scan *sc);
  * labels/label_off: CSR of each query's scan-key labels, label_off == NULL = no key.
  * out_tid [B*k] (block<<16|offset, DANN_INVALID_TID past out_count[b]), out_dist [B*k],
  * out_count [B] rows produced, out_stats [B] (each may be NULL except out_tid).
- * rescore + k is bounded by the rerank kernel's shared memory (about 45 000 rows at 768 dimensions):
- * larger requests return DANN_ERR_INVALID_ARG (the streaming scan operator is not bound by the rerank window). */
+ * rescore + k is bounded by the rerank kernel's shared memory (on a B200 about 57 000 rows at 768 dimensions,
+ * 42 000 at 16 000): larger requests return DANN_ERR_INVALID_ARG and leave the handle usable (the streaming
+ * scan operator is not bound by the rerank window). */
 int dann_search_batch(dann_index *ix, const float *queries, const int16_t *labels,
                       const int32_t *label_off, int B, int k, int search_list_size,
                       int rescore, uint64_t *out_tid, float *out_dist, uint32_t *out_count,
@@ -190,7 +191,9 @@ int dann_full_distance(dann_index *ix, const float *d_q_full, const uint32_t *d_
  * the reference's way: a label-filtered insertion pass from the label start nodes, then the unfiltered
  * one (graph/mod.rs:637-660), with the label-aware prune (:445-455).  On return every list holds
  * <= num_neighbors ids.  The graph is a valid diskann graph but not the reference's serial insertion
- * order, so it serves bulk builds, fixtures and benchmarks. */
+ * order, so it serves bulk builds, fixtures and benchmarks.  The prune step stages 128 candidate codes per
+ * warp in shared memory, which on a B200 holds codes of up to 222 words (14 208 dimensions at 1 bit); a wider
+ * code returns DANN_ERR_CAPACITY before anything is written, and the index keeps its neighbour lists. */
 typedef struct {
     uint32_t batches;
     float search_ms, prune_ms, sort_ms, backlink_ms, total_ms;

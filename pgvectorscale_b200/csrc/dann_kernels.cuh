@@ -301,7 +301,9 @@ __global__ void __launch_bounds__(128) dann_rerank_kernel(const RerankArgs a) {
     const uint32_t dim4 = (ix.dim + 3u) & ~3u;
     float *ds = qs + dim4;                                              /* [c_target] */
     uint64_t *hp = reinterpret_cast<uint64_t *>(ds + ((a.c_target + 1u) & ~1u)); /* [rescore] */
-    DANN_STATIC_SMEM uint64_t bar;
+    /* the TMA barrier lives in the dynamic window too: with no static shared memory the host's check of a request
+     * against the opt-in limit (rerank_smem_bytes) is exact */
+    uint64_t *bar = hp + a.rescore;
     const int q = blockIdx.x;
     const uint32_t sl = a.stream_len[q];
     const uint32_t *st = a.stream + (size_t)q * a.c_target;
@@ -319,7 +321,7 @@ __global__ void __launch_bounds__(128) dann_rerank_kernel(const RerankArgs a) {
         return;
     }
 
-    stage_query_row(qs, a.q_full + (size_t)q * ix.dim, ix.dim, &bar);
+    stage_query_row(qs, a.q_full + (size_t)q * ix.dim, ix.dim, bar);
     {
         const uint32_t lane = threadIdx.x & 31, mm = lane & 7, gbase = lane & 24;
         const uint32_t group = threadIdx.x >> 3, ngroups = blockDim.x >> 3;

@@ -742,6 +742,13 @@ static int run_search(dann_index *ix, const uint64_t *d_q_codes, const int16_t *
     return DANN_OK;
 }
 
+/* dann_rerank_kernel's dynamic shared memory: the query row, one f32 per streamed row (even count, so that the window
+ * is 8-byte aligned), the rescore window, the TMA barrier (16 B), and the slack.  Both the request check and the launch
+ * use it, so that a request the check accepts always launches. */
+static size_t rerank_smem_bytes(uint32_t dim, uint32_t c_target, uint32_t rescore) {
+    return (size_t)((dim + 3u) & ~3u) * 4 + (size_t)((c_target + 1u) & ~1u) * 4 + (size_t)rescore * 8 + 16 + DANN_SMEM_SLACK;
+}
+
 /* B queries, first k rows each.  All pointers are device pointers. */
 static int search_batch_device_locked(dann_index *ix, const float *d_queries, const int16_t *d_labels,
                                       const int32_t *d_label_off, int B, int k, int L, int rescore,
@@ -752,12 +759,6 @@ static int search_batch_device_locked(dann_index *ix, const float *d_queries, co
     if (L < 1 || L > 10000) return fail(DANN_ERR_INVALID_ARG, "search_list_size %d outside 1..10000 (guc.rs:11-26)", L);
     if (rescore < 0 || rescore > 1000) return fail(DANN_ERR_INVALID_ARG, "rescore %d outside 0..1000 (guc.rs:28-43)", rescore);
     if (!d_queries || !d_out_tid) return fail(DANN_ERR_INVALID_ARG, "NULL query or output buffer");
-    {   /* the rerank kernel keeps one f32 per streamed row + the window in shared memory */
-        const size_t need_smem = (size_t)((v.dim + 3u) & ~3u) * 4 + ((size_t)rescore + (size_t)k + 2) * 4 + (size_t)rescore * 8 + 64;
-        if (need_smem > ix->smem_optin)
-            return fail(DANN_ERR_INVALID_ARG, "k=%d rows with rescore=%d need %zu B of shared memory per scan (limit %zu): "
-                        "fetch fewer rows per scan", k, rescore, need_smem, ix->smem_optin);
-    }
     if (ix->plain) {
         if (d_label_off) return fail(DANN_ERR_INVALID_ARG, "plain storage does not support label filters (plain/storage.rs:260)");
         /* scan.rs:392-403: a plain index only resorts when it holds fewer dimensions than the heap column */
@@ -766,6 +767,10 @@ static int search_batch_device_locked(dann_index *ix, const float *d_queries, co
     if (rescore > 0 && v.n && !v.vectors) return fail(DANN_ERR_STATE, "index has no heap vectors yet (dann_index_set_vectors): rescore must be 0");
     /* rows needed from the approximate stream: scan.rs:255-305 */
     const uint32_t c_target = rescore == 0 ? (uint32_t)k : (uint32_t)rescore + (uint32_t)k - 1u;
+    const size_t rerank_smem = rerank_smem_bytes(v.dim, c_target, (uint32_t)rescore);
+    if (rerank_smem > ix->smem_optin) /* the rerank kernel keeps one f32 per streamed row + the window in shared memory */
+        return fail(DANN_ERR_INVALID_ARG, "k=%d rows with rescore=%d need %zu B of shared memory per scan (limit %zu): "
+                    "fetch fewer rows per scan", k, rescore, rerank_smem, ix->smem_optin);
 
     CK(ix->sc_qfull.reserve((size_t)B * v.dim * sizeof(float)));
     CK(ix->sc_qcodes.reserve((size_t)B * v.cw * sizeof(uint64_t)));
@@ -809,10 +814,9 @@ static int search_batch_device_locked(dann_index *ix, const float *d_queries, co
     r.out_node = d_out_node;
     r.out_count = d_out_count;
     r.stats = d_stats;
-    size_t smem = (size_t)((v.dim + 3u) & ~3u) * 4 + (size_t)((c_target + 1u) & ~1u) * 4 + (size_t)rescore * 8 + 16 + DANN_SMEM_SLACK;
-    if (smem > 48 * 1024)
-        CK(cudaFuncSetAttribute(dann_rerank_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    dann_rerank_kernel<<<B, 128, smem, st>>>(r);
+    if (rerank_smem > 48 * 1024)
+        CK(cudaFuncSetAttribute(dann_rerank_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rerank_smem));
+    dann_rerank_kernel<<<B, 128, rerank_smem, st>>>(r);
     ix->launches++;
     CK(cudaGetLastError());
     if (ix->plain && rescore > 0) {
@@ -1002,6 +1006,14 @@ extern "C" int dann_build_graph(dann_index *ix, int num_neighbors, int search_li
     const uint32_t n = v.n;
     const uint32_t vis_cap = 2 * DANN_BUILD_CMAX;
     const uint32_t mb = std::min<uint32_t>(max_batch, n);
+    /* the prune kernel stages DANN_BUILD_CMAX candidate codes per warp in shared memory: a code too wide for one warp is
+     * refused here, before the neighbour lists are cleared, so that a refused build leaves the index as it was */
+    const uint32_t cws = v.cw | 1u;
+    const size_t pw = ((size_t)DANN_BUILD_CMAX * 8 + (size_t)DANN_BUILD_CMAX * cws * 8 + DANN_BUILD_CMAX * 4 +
+                       DANN_BUILD_SLACK * 4 + DANN_BUILD_SLACK * 2 + 15) & ~(size_t)15;
+    const size_t budget = ix->smem_optin > 1024 ? ix->smem_optin - 1024 : ix->smem_optin;
+    const int bw = (int)std::min<size_t>(8, budget / pw);
+    if (bw < 1) return fail(DANN_ERR_CAPACITY, "SBQ code of %u words is too wide for the prune kernel's shared memory", v.words);
 
     DevBuf b_dist, b_deg, b_vis, b_vlen, b_k0, b_k1, b_v0, b_v1, b_heads, b_tmp, b_stream, b_slen, b_stats;
     struct Cleanup {
@@ -1036,7 +1048,7 @@ extern "C" int dann_build_graph(dann_index *ix, int num_neighbors, int search_li
     BuildArgs ba;
     ba.codes = v.codes;
     ba.cw = v.cw;
-    ba.cws = v.cw | 1u;
+    ba.cws = cws;
     ba.n = n;
     ba.nbrs = nbrs;
     ba.nbr_dist = b_dist.as<uint16_t>();
@@ -1046,12 +1058,7 @@ extern "C" int dann_build_graph(dann_index *ix, int num_neighbors, int search_li
     ba.max_alpha = max_alpha;
     ba.label_off = v.has_labels ? v.label_off : nullptr;
     ba.labels = v.has_labels ? v.labels : nullptr;
-    const size_t pw = ((size_t)DANN_BUILD_CMAX * 8 + (size_t)DANN_BUILD_CMAX * ba.cws * 8 + DANN_BUILD_CMAX * 4 +
-                       DANN_BUILD_SLACK * 4 + DANN_BUILD_SLACK * 2 + 15) & ~(size_t)15;
     ba.per_warp_smem = (uint32_t)pw;
-    const size_t budget = ix->smem_optin > 1024 ? ix->smem_optin - 1024 : ix->smem_optin;
-    int bw = (int)std::min<size_t>(8, budget / pw);
-    if (bw < 1) return fail(DANN_ERR_CAPACITY, "SBQ code of %u words is too wide for the prune kernel's shared memory", v.words);
     const size_t bsmem = pw * bw + DANN_SMEM_SLACK;
     CK(cudaFuncSetAttribute(dann_build_prune_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem));
     CK(cudaFuncSetAttribute(dann_build_backlink_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem));

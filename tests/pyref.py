@@ -107,6 +107,8 @@ def quantize(v, bits, mean, m2, count, words):
                 ones = 0
             elif np.isnan(idx):
                 ones = 0
+            elif np.isinf(idx):     # constant dimension (m2 = 0), query above its value: `inf as usize` saturates
+                ones = bits
             else:
                 ones = min(int(math.floor(float(idx))), bits)
         for j in range(ones):

@@ -40,8 +40,9 @@ def _run(files, extra_env=None, workers=4, timeout=1500, asan=False):
 def test_gpu_parity_suite_passes_under_emulation():
     passed, out = _run(["tests/test_gpu_parity.py", "tests/test_zz_c_harness_gpu.py", "tests/test_zz_d_build_small_gpu.py",
                         "tests/test_zz_e_coalescer_gpu.py", "tests/test_zz_f_fuzz_gpu.py",
-                        "tests/test_zz_g_oom_paths_emulated.py", "tests/test_zz_h_two_rank_emulated.py"])
-    assert passed >= 97 and "skipped" not in out.splitlines()[-1], out[-500:]
+                        "tests/test_zz_g_oom_paths_emulated.py", "tests/test_zz_h_two_rank_emulated.py",
+                        "tests/test_zz_l_wide_codes_gpu.py"])
+    assert passed >= 97 + 45 and "skipped" not in out.splitlines()[-1], out[-500:]
 
 
 def test_two_replica_group_under_emulation():
